@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          our CUDA path
     python bench.py --impl reference [...]                        the reference's CPU path
+    python bench.py --dump-outputs DIR [...]                      also write what the last timed step returned, DIR/<name>.npy
 
 Workload (BASELINE.json configs[1], the configuration the metric is quoted on):
 fused block_extractor + local_attn_reshape + softmax ("ExtractorAttn tail",
@@ -205,6 +206,23 @@ def bind_to_gpu_numa_node(torch, local_rank):
         return None
 
 
+DUMP_SAMPLE = 1 << 21      # elements kept of a larger output: the four outputs of the cfg2 step take 32 MB in float32
+
+
+def sample_outputs(torch, named):
+    """{name: float32 numpy array} of the step's outputs, in logical [B,C,H,W] order whatever the storage; an output with
+    more than DUMP_SAMPLE elements is reduced to the same DUMP_SAMPLE seeded positions (sorted) on every run"""
+    res = {}
+    for name, t in named.items():
+        flat = t.detach().reshape(-1)
+        if flat.numel() > DUMP_SAMPLE:
+            g = torch.Generator(device="cpu").manual_seed(0)
+            idx = torch.randint(0, flat.numel(), (DUMP_SAMPLE,), generator=g).sort().values
+            flat = flat[idx.to(flat.device)]
+        res[name] = flat.float().cpu().numpy()
+    return res
+
+
 def _time(torch, fn, warm, n):
     for _ in range(warm):
         fn()
@@ -333,7 +351,14 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra keys (iid flow, cfg3 resample2d, reference CUDA kernels)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (out, grad_source, grad_flow, grad_logits of rank 0) as "
+                         f"DIR/<name>.npy in float32; an output above {DUMP_SAMPLE} elements is a fixed seeded sample of it")
     args = ap.parse_args()
+    if args.dump_outputs is not None:
+        if args.workload != "cfg2" or args.impl != "ours":
+            ap.error("--dump-outputs covers the default workload on the GPU (--workload cfg2 --impl ours)")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -421,11 +446,19 @@ def main():
     barrier()
     t_wall0 = time.time()
     launches0 = _lib.lib().gfla_debug_launch_count()
+    last = None
     for i in range(steps):
-        step(ev[i])
+        last = None            # the previous step's outputs are freed before the next step, as if they were discarded
+        last = step(ev[i])
     launches = int(_lib.lib().gfla_debug_launch_count() - launches0)   # kernels of libgfla_warp.so launched in the timed region
     barrier()
     t_wall1 = time.time()
+    dump = None
+    if args.dump_outputs is not None and rank == 0:
+        out, (gs, gf, gl) = last
+        dump = sample_outputs(torch, {"out": out, "grad_source": gs, "grad_flow": gf, "grad_logits": gl})
+        del out, gs, gf, gl
+    del last
     total_ms = ev[0][0].elapsed_time(ev[-1][2])
     fwd_ms = sum(e[0].elapsed_time(e[1]) for e in ev) / steps
     bwd_ms = sum(e[1].elapsed_time(e[2]) for e in ev) / steps
@@ -445,7 +478,7 @@ def main():
             step_planar()
         barrier()
         a_, b__ = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        p_steps = max(steps, 20)
+        p_steps = steps
         a_.record()
         for _ in range(p_steps):
             step_planar()
@@ -511,6 +544,10 @@ def main():
                "chunks": len(chunks), "streams": len(side), "pipelined_across_steps": True}
     if rank == 0:
         sampler.stop()
+    if dump is not None:
+        import numpy as np
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     if rank != 0:
         if world > 1:

@@ -27,7 +27,9 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 import oracle.oracle as orc  # noqa: E402
+from conftest import FixedFeatures, golden_grad_out, perceptual_inputs, sample_index, sha256  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
 
@@ -55,7 +57,7 @@ def main():
         ("gradcheck_shape", np.float64, 4, 6, 14, 10, 14, 10, 3, "rand1.8"),  # test_block_extractor.py:74-78
         ("k2", np.float64, 1, 2, 6, 5, 6, 5, 2, "iid8"),
     ]
-    for name, dt, B, C, Hs, Ws, Hf, Wf, k, kind in cases:
+    for seed, (name, dt, B, C, Hs, Ws, Hf, Wf, k, kind) in enumerate(cases):
         src = rng.standard_normal((B, C, Hs, Ws)).astype(dt)
         if kind == "iid8":
             flow = rng.uniform(-8, 8, (B, 2, Hf, Wf))
@@ -71,10 +73,13 @@ def main():
             flow = rng.uniform(0, 1, (B, 2, Hf, Wf)) * 1.8
         flow = np.ascontiguousarray(flow.astype(dt))
         out = R.block_extract_fwd(src, flow, k)
-        gout = rng.standard_normal(out.shape).astype(dt)
+        # out and grad_out are k*k times the size of the source, so neither is stored: out is compared bit for bit and
+        # its digest stands in for it; grad_out comes from a stored seed (conftest.load_golden rebuilds it)
+        rng.standard_normal(out.shape)      # an unused draw that keeps the later sections' inputs as committed
+        gout = golden_grad_out(seed, out.shape, dt)
         gs, gf = R.block_extract_bwd(src, flow, gout, k)
-        for key, v in dict(source=src, flow=flow, out=out, grad_out=gout, grad_source=gs, grad_flow=gf,
-                           k=np.int32(k)).items():
+        for key, v in dict(source=src, flow=flow, out_sha256=np.str_(sha256(out)), grad_out_seed=np.int64(seed),
+                           grad_out_shape=np.array(out.shape, np.int64), grad_source=gs, grad_flow=gf, k=np.int32(k)).items():
             be[f"{name}/{key}"] = v
     np.savez_compressed(os.path.join(OUT, "block_extractor.npz"), **be)
 
@@ -142,9 +147,170 @@ def main():
             la[f"{name}/{key}"] = v
     np.savez_compressed(os.path.join(OUT, "local_attn.npz"), **la)
 
+    oracle_vs_ref(R)
+    reference_fullsize(R)
+    reference_losses(R)
+    reference_perceptual(R)
+
     for f in sorted(os.listdir(OUT)):
         if f.endswith(".npz"):
             print(f, os.path.getsize(os.path.join(OUT, f)), "bytes")
+
+
+def oracle_vs_ref(R):
+    """digests of the reference's outputs on tests/test_oracle_vs_ref.py's inputs (one thread, like the oracle)"""
+    import test_oracle_vs_ref as T
+
+    ref = {}
+
+    def keep(name, outputs):
+        for key, a in outputs.items():
+            ref[f"{name}/{key}"] = np.str_(sha256(a))
+
+    for dt in (np.float32, np.float64):
+        for shape in T.BLOCK_SHAPES:
+            keep(T.case_name("block_extractor", np.dtype(dt).name, *shape), T.block_outputs(R, dt, shape))
+        for cfg in T.RESAMPLE_CFGS:
+            keep(T.case_name("resample2d", np.dtype(dt).name, *cfg), T.resample_outputs(R, dt, cfg))
+    for k in T.RESHAPE_KS:
+        keep(T.case_name("reshape", k), T.reshape_outputs(R, k))
+    np.savez_compressed(os.path.join(OUT, "oracle_vs_ref.npz"), **ref)
+
+
+def reference_fullsize(R):
+    """tests/test_gpu_refcuda.py's full-size cases (BASELINE configs 2 and 3): the reference's outputs at the fixed
+    sample of positions, plus each output's largest magnitude (the tests' relative tolerances scale with it).  All host
+    threads: the order of the atomic adds into grad_flow, and so its last bits (~1e-6 relative), vary from run to run."""
+    import test_gpu_refcuda as T
+    from oracle.ref_pipeline import local_attn_fwd_bwd
+
+    R.set_threads(os.cpu_count() or 1)
+    host = lambda *ts: [np.ascontiguousarray(t.numpy()) for t in ts]
+    ref = {}
+
+    def keep(case, **arrays):
+        for name, a in arrays.items():
+            ref[f"{case}/{name}"] = a.reshape(-1)[sample_index(a.size)].astype(np.float32)
+            ref[f"{case}/{name}_absmax"] = np.float64(np.abs(a).max())
+
+    for case in ("tile_smooth", "tile_iid", "planar", "fp32", "host"):
+        inputs, k = T.cfg2_case(case, device="cpu")
+        per_sample = [local_attn_fwd_bwd(R, *host(*(t[b:b + 1] for t in inputs)), k) for b in range(inputs[0].shape[0])]
+        out, _, gs, gf, gl = (np.concatenate(parts) for parts in zip(*per_sample))
+        keep(case, out=out, grad_source=gs, grad_flow=gf, grad_logits=gl)
+    (src, flow, go), k = T.block_extractor_case(device="cpu")
+    src, flow, go = host(src, flow, go)
+    out = R.block_extract_fwd(src, flow, k)
+    keep("block_extractor", out=out)
+    del out
+    gs, gf = R.block_extract_bwd(src, flow, go, k)
+    keep("block_extractor", grad_source=gs, grad_flow=gf)
+    for ks, sigma in ((2, 5.0), (4, 2.0)):
+        (x, in2, go), _ = T.resample2d_case(ks, sigma, device="cpu")
+        x, in2, go = host(x, in2, go)
+        g1, g2 = R.resample2d_bwd(x, in2, go, ks, 1)
+        keep(f"resample2d_ks{ks}", out=R.resample2d_fwd(x, in2, ks, 1), grad_in1=g1, grad_in2=g2)
+    R.set_threads(1)
+    np.savez_compressed(os.path.join(OUT, "reference_fullsize.npz"), **ref)
+
+
+def reference_external_function():
+    """the reference's model/networks/external_function.py on this package's ops (compat.install), importable here"""
+    import types
+    import gfla_b200
+    from baseline import snapshot
+    snapshot.snapshot()
+    gfla_b200.compat.install(reference_root=snapshot.root())
+    util = types.ModuleType("util")                   # external_function.py:8 (visualisation helpers, not needed here)
+    util.util = types.ModuleType("util.util")
+    sys.modules.setdefault("util", util)
+    sys.modules.setdefault("util.util", util.util)
+    from model.networks import external_function as ef
+    return ef
+
+
+def reference_losses(R):
+    """what the reference's own AffineRegularizationLoss / MultiAffineRegularizationLoss classes compute
+    (tests/test_reference_integration.py): the kernel per kz, flow2grid of a seeded flow, the layer order and kernel
+    sizes; and (tests/test_gpu_models.py) the loss and its flow gradient on a seeded flow, with the two custom ops of
+    the class on the reference's kernel bodies"""
+    from oracle.ref_pipeline import make_functions
+    ExtractFn, ReshapeFn = make_functions(R)
+
+    class HostBlockExtractor(torch.nn.Module):
+        def __init__(self, kz):
+            super().__init__()
+            self.kz = kz
+
+        def forward(self, source, flow_field):
+            return ExtractFn.apply(source.contiguous(), flow_field.contiguous(), self.kz)
+
+    class HostLocalAttnReshape(torch.nn.Module):
+        def forward(self, inputs, kernel_size):
+            return ReshapeFn.apply(inputs.contiguous(), kernel_size)
+
+    ef = reference_external_function()
+    out = {}
+    for kz in (3, 4, 5):
+        loss = ef.AffineRegularizationLoss(kz)
+        flow = torch.randn(2, 2, 9, 11, generator=torch.Generator().manual_seed(kz))
+        out[f"kz{kz}/kernel"] = loss.kernel.numpy()
+        out[f"kz{kz}/flow"], out[f"kz{kz}/grid"] = flow.numpy(), loss.flow2grid(flow).numpy()
+        if kz != 4:
+            loss.extractor, loss.reshape = HostBlockExtractor(kz), HostLocalAttnReshape()
+            flow = (torch.randn(2, 2, 32, 32, generator=torch.Generator().manual_seed(kz)) * 3).requires_grad_()
+            value = loss(flow)
+            value.backward()
+            out[f"kz{kz}/loss"], out[f"kz{kz}/loss_grad"] = np.float64(value.item()), flow.grad.numpy()
+    m = ef.MultiAffineRegularizationLoss({"2": 5, "3": 3})
+    out["multi/layers"] = np.array([int(x) for x in m.layers], np.int64)
+    out["multi/kz"] = np.array([m.method_dic[x].kz for x in m.layers], np.int64)
+    np.savez_compressed(os.path.join(OUT, "reference_losses.npz"), **out)
+
+
+def reference_perceptual(R):
+    """the reference's PerceptualCorrectness on conftest.perceptual_inputs with conftest.FixedFeatures as its feature
+    extractor: loss and flow gradients, without and with the mask, through its grid_sample branch ("bilinear",
+    tests/test_losses.py) and through its Resample2d(4, 1, sigma=2) branch ("resample", tests/test_gpu_resample_cosine.py),
+    whose op runs on the reference's kernel bodies on the host"""
+    import torchvision
+    ef = reference_external_function()
+
+    class HostResample2dFn(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, in1, in2):
+            ctx.save_for_backward(in1, in2)
+            return torch.from_numpy(R.resample2d_fwd(in1.detach().numpy(), in2.detach().numpy(), 4, 1))
+
+        @staticmethod
+        def backward(ctx, g):
+            in1, in2 = ctx.saved_tensors
+            g1, g2 = R.resample2d_bwd(in1.detach().numpy(), in2.detach().numpy(), np.ascontiguousarray(g.numpy()), 4, 1)
+            return torch.from_numpy(g1), torch.from_numpy(g2)
+
+    class HostResample2d(torch.nn.Module):      # resample2d.py:43-51: sigma appended as a third flow channel
+        def forward(self, input1, input2):
+            b, _, h, w = input2.shape
+            return HostResample2dFn.apply(input1.contiguous(), torch.cat([input2, torch.full((b, 1, h, w), 2.0)], 1).contiguous())
+
+    vgg19 = torchvision.models.vgg19
+    torchvision.models.vgg19 = lambda pretrained=False, **kw: vgg19(weights=None)     # built, then replaced: no weights needed
+    try:
+        loss = ef.PerceptualCorrectness()
+    finally:
+        torchvision.models.vgg19 = vgg19
+    loss.vgg, loss.resample = FixedFeatures(), HostResample2d()
+    target, source, mask, flows = perceptual_inputs()
+    out = {}
+    for branch in ("bilinear", "resample"):
+        for name, m in (("nomask", None), ("mask", mask)):
+            fs = [f.clone().requires_grad_() for f in flows]
+            value = loss(target, source, fs, [2, 3], m, branch == "bilinear")
+            value.backward()
+            out[f"{branch}_{name}/loss"] = np.float64(value.item())
+            for i, f in enumerate(fs):
+                out[f"{branch}_{name}/grad{i}"] = f.grad.numpy()
+    np.savez_compressed(os.path.join(OUT, "reference_perceptual.npz"), **out)
 
 
 if __name__ == "__main__":

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -42,3 +44,27 @@ def test_reference_arm_other_ranks_stay_silent():
     r = _run({"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2", "MASTER_ADDR": "127.0.0.1", "MASTER_PORT": "29591"})
     assert r.returncode == 0, r.stderr[-2000:]
     assert not [l for l in r.stdout.splitlines() if l.startswith("{")]
+
+
+def test_dump_outputs_is_refused_outside_the_gpu_arm(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, cwd=ROOT, timeout=300)
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_step(tmp_path):
+    """--dump-outputs: the four arrays the timed step returns, float32, within 64 MB; --steps sets the timed steps"""
+    import numpy as np
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--no-extras", "--no-e2e",
+                        "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, cwd=ROOT, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    j = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+    assert j["steps"] == 2 and j["gpu_launches"] == 2 * 2          # one fused forward + one fused backward per step
+    files = sorted(p.name for p in tmp_path.iterdir())
+    assert files == ["grad_flow.npy", "grad_logits.npy", "grad_source.npy", "out.npy"]
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 << 20
+    arrays = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+    assert all(a.dtype == np.float32 and np.isfinite(a).all() for a in arrays.values())
+    assert arrays["grad_flow"].size == 16 * 2 * 256 * 256                 # small enough to be written whole
+    assert arrays["out"].std() > 0 and arrays["grad_source"].std() > 0

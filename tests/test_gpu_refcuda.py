@@ -1,18 +1,23 @@
-"""GPU (-m gpu): parity against the REFERENCE'S OWN kernels on the GPU box.
+"""GPU (-m gpu): parity against the REFERENCE'S OWN kernels at BASELINE.json's full sizes.
 
-Two reference builds travel with the snapshot (git-ignored, built by ``__graft_entry__.build()`` where
-/root/reference exists):
+The `<5,256>` tile instantiations that bench.py times are checked at 256x256, C=256, k=5 -- forward and
+backward -- against the reference itself, not only against our own kernels.  What the reference computed on
+these seeded inputs (its kernel bodies compiled for the host, oracle/_ref, composed like its ExtractorAttn) is
+stored in tests/golden/reference_fullsize.npz by tests/golden/make_golden.py: each output at the same fixed
+sample of positions (conftest.sample_index) plus its largest magnitude.  Tolerances = north_star: 1e-4 fp32,
+1e-2 bf16 (absolute, flat).
+
+test_refcuda_equals_host_reference checks the two builds of the reference's kernel text against each other:
   * ``oracle/_ref/libgfla_ref.so``       -- the reference kernel bodies compiled for the host (OpenMP);
   * ``oracle/_ref/libgfla_ref_cuda.so``  -- the same extracted text compiled by nvcc for sm_100a
     (``oracle/ref_cuda*.cu``: plain launchers, no ATen) = "the reference's CUDA kernels, recompiled".
-The CUDA build reaches BASELINE.json's full sizes in milliseconds, so the `<5,256>` tile instantiations
-that bench.py times are checked here at 256x256, C=256, k=5 -- forward and backward -- against the reference
-itself (chunked, because the reference's `int n` overflows above B=5 at this size), not only against
-our own kernels.  Tolerances = north_star: 1e-4 fp32, 1e-2 bf16 (absolute, flat).
+Both are built by ``__graft_entry__.build()`` only where a checkout of the reference exists; it skips elsewhere.
 """
 import numpy as np
 import pytest
 import torch
+
+from conftest import load_golden, sample_index
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -35,19 +40,70 @@ def F_():
     return gfla_b200.functional
 
 
-def _smooth_flow(B, H, W, amp=8.0, seed=0):
+def _smooth_flow(B, H, W, amp=8.0, seed=0, device=DEV):
     g = torch.Generator(device="cpu").manual_seed(seed)
     coarse = torch.rand(B, 2, max(H // 16, 2), max(W // 16, 2), generator=g) * 2 * amp - amp
-    return torch.nn.functional.interpolate(coarse, size=(H, W), mode="bilinear", align_corners=True).to(DEV).contiguous()
+    return torch.nn.functional.interpolate(coarse, size=(H, W), mode="bilinear", align_corners=True).to(device).contiguous()
 
 
-def _inputs(B, C, H, W, k, kind, seed):
+def _inputs(B, C, H, W, k, kind, seed, device=DEV):
     g = torch.Generator(device="cpu").manual_seed(seed)
-    src = torch.randn(B, C, H, W, generator=g).to(DEV)
-    logits = torch.randn(B, k * k, H, W, generator=g).to(DEV)
-    gout = torch.randn(B, C, H, W, generator=g).to(DEV)
-    flow = _smooth_flow(B, H, W, seed=seed) if kind == "smooth" else ((torch.rand(B, 2, H, W, generator=g) * 16 - 8).to(DEV))
+    src = torch.randn(B, C, H, W, generator=g).to(device)
+    logits = torch.randn(B, k * k, H, W, generator=g).to(device)
+    gout = torch.randn(B, C, H, W, generator=g).to(device)
+    flow = _smooth_flow(B, H, W, seed=seed, device=device) if kind == "smooth" else ((torch.rand(B, 2, H, W, generator=g) * 16 - 8).to(device))
     return src, flow, logits, gout
+
+
+# inputs of the full-size cases, on `device` (tests/golden/make_golden.py builds them on the host)
+def cfg2_case(name, device=DEV):
+    """-> (inputs in the dtype the reference ran on, k); the bf16 cases hand the reference the bf16-rounded values"""
+    B, kind, seed, bf16 = {"tile_smooth": (2, "smooth", 21, True), "tile_iid": (2, "iid", 21, True), "planar": (1, "smooth", 22, True),
+                           "fp32": (1, "smooth", 23, False), "host": (1, "smooth", 24, True)}[name]
+    src, flow, logits, gout = _inputs(B, 256, 256, 256, 5, kind, seed, device)
+    if bf16:
+        src, logits, gout = (t.bfloat16().float() for t in (src, logits, gout))
+    return (src, flow, logits, gout), 5
+
+
+def block_extractor_case(device=DEV):
+    B, C, H, W, k = 1, 256, 256, 256, 5
+    src, flow, _, _ = _inputs(B, C, H, W, k, "smooth", seed=25, device=device)
+    go = torch.randn(B, C, k * H, k * W, generator=torch.Generator(device="cpu").manual_seed(26)).to(device)
+    return (src, flow, go), k
+
+
+def resample2d_case(ks, sigma, device=DEV):
+    B, C, H, W = 2, 128, 512, 512
+    g = torch.Generator(device="cpu").manual_seed(31)
+    x = torch.randn(B, C, H, W, generator=g).to(device)
+    go = torch.randn(B, C, H, W, generator=g).to(device)
+    in2 = torch.cat([_smooth_flow(B, H, W, seed=3, device=device), torch.full((B, 1, H, W), sigma, device=device)], 1).contiguous()
+    return (x, in2, go), ks
+
+
+@pytest.fixture(scope="module")
+def REF():
+    return load_golden("reference_fullsize")
+
+
+class _Ref:
+    """one case of the stored reference outputs: ref[name] = sampled values on the GPU, ref.absmax(name) = max |value|"""
+
+    def __init__(self, case):
+        self.case = case
+
+    def __getitem__(self, name):
+        return torch.from_numpy(self.case[name]).to(DEV)
+
+    def absmax(self, name):
+        return float(self.case[name + "_absmax"])
+
+
+def _at(t):
+    """t (any storage order) at the stored positions of its logical C-order flattening, as float32"""
+    flat = t.detach().float().reshape(-1)
+    return flat[torch.from_numpy(sample_index(flat.numel())).to(flat.device)]
 
 
 # ----------------------------------------------------------------------------- the checker itself: nvcc build == host build
@@ -76,104 +132,85 @@ def test_refcuda_equals_host_reference(RC, ref_lib, k):
 
 # ----------------------------------------------------------------------------- full-size cfg2 samples vs the reference's kernels
 @pytest.mark.parametrize("kind", ["smooth", "iid"])
-def test_cfg2_fullsize_tile_path_vs_reference_cuda(RC, F_, kind):
+def test_cfg2_fullsize_tile_path_vs_reference_cuda(REF, F_, kind):
     """B=2, C=256, 256x256, k=5, bf16 channels_last -- exactly the <5,256> kernels of the bench step (strip forward,
-    tile backward) -- vs the reference's unfused pipeline on its own CUDA kernels in fp32 on the bf16-rounded inputs"""
-    B, C, H, W, k = 2, 256, 256, 256, 5
-    src, flow, logits, gout = _inputs(B, C, H, W, k, kind, seed=21)
+    tile backward) -- vs the reference's unfused pipeline in fp32 on the bf16-rounded inputs"""
+    (src, flow, logits, gout), k = cfg2_case(f"tile_{kind}")
+    ref = _Ref(REF[f"tile_{kind}"])
     sb, lb, gb = src.bfloat16(), logits.bfloat16(), gout.bfloat16()
-    ref_out, ref_gs, ref_gf, ref_gl = RC.local_attn_fwd_bwd(sb.float(), flow, lb.float(), gb.float(), k, chunk=1)
     s_cl, g_cl = sb.contiguous(memory_format=CL), gb.contiguous(memory_format=CL)
     out = F_.local_attn_fwd(s_cl, flow, lb, k, algo="tile")
     gs, gf, gl = F_.local_attn_bwd(s_cl, flow, lb, g_cl, k, algo="tile")
-    assert (out.float() - ref_out).abs().max().item() <= 1e-2
-    assert (gs.float() - ref_gs).abs().max().item() <= 1e-2                      # flat, like north_star
-    assert (gs.float() - ref_gs).abs().max().item() <= 1e-2 * max(1.0, ref_gs.abs().max().item())
-    assert (gl.float() - ref_gl).abs().max().item() <= 1e-2
+    assert (_at(out) - ref["out"]).abs().max().item() <= 1e-2
+    assert (_at(gs) - ref["grad_source"]).abs().max().item() <= 1e-2                      # flat, like north_star
+    assert (_at(gs) - ref["grad_source"]).abs().max().item() <= 1e-2 * max(1.0, ref.absmax("grad_source"))
+    assert (_at(gl) - ref["grad_logits"]).abs().max().item() <= 1e-2
     # grad_flow sums C*k*k products of O(1) terms: bf16 inputs are exact here, the difference is summation order / Q in fp32
-    assert (gf - ref_gf).abs().max().item() <= 1e-2 * max(1.0, ref_gf.abs().max().item())
+    assert (_at(gf) - ref["grad_flow"]).abs().max().item() <= 1e-2 * max(1.0, ref.absmax("grad_flow"))
     # error histogram of grad_source (the bf16 reduce-add path): how far from the bound the bulk sits
-    err = (gs.float() - ref_gs).abs()
+    err = (_at(gs) - ref["grad_source"]).abs()
     assert err.mean().item() <= 1e-3
 
 
-def test_cfg2_fullsize_planar_nchw_vs_reference_cuda(RC, F_):
+def test_cfg2_fullsize_planar_nchw_vs_reference_cuda(REF, F_):
     """the reference's own contiguous-NCHW contract at full size (forward NCHW tile kernel, backward through the tile kernels)"""
-    B, C, H, W, k = 1, 256, 256, 256, 5
-    src, flow, logits, gout = _inputs(B, C, H, W, k, "smooth", seed=22)
+    (src, flow, logits, gout), k = cfg2_case("planar")
+    ref = _Ref(REF["planar"])
     sb, lb, gb = src.bfloat16(), logits.bfloat16(), gout.bfloat16()
-    ref_out, ref_gs, ref_gf, ref_gl = RC.local_attn_fwd_bwd(sb.float(), flow, lb.float(), gb.float(), k, chunk=1)
     out = F_.local_attn_fwd(sb, flow, lb, k)
     gs, gf, gl = F_.local_attn_bwd(sb, flow, lb, gb, k)
     assert out.is_contiguous() and gs.is_contiguous()
-    assert (out.float() - ref_out).abs().max().item() <= 1e-2
-    assert (gs.float() - ref_gs).abs().max().item() <= 1e-2
-    assert (gl.float() - ref_gl).abs().max().item() <= 1e-2
-    assert (gf - ref_gf).abs().max().item() <= 1e-2 * max(1.0, ref_gf.abs().max().item())
+    assert (_at(out) - ref["out"]).abs().max().item() <= 1e-2
+    assert (_at(gs) - ref["grad_source"]).abs().max().item() <= 1e-2
+    assert (_at(gl) - ref["grad_logits"]).abs().max().item() <= 1e-2
+    assert (_at(gf) - ref["grad_flow"]).abs().max().item() <= 1e-2 * max(1.0, ref.absmax("grad_flow"))
 
 
-def test_cfg2_fullsize_fp32_vs_reference_cuda(RC, F_):
+def test_cfg2_fullsize_fp32_vs_reference_cuda(REF, F_):
     """fp32 (the reference's dtype), one full-size sample: 1e-4"""
-    B, C, H, W, k = 1, 256, 256, 256, 5
-    src, flow, logits, gout = _inputs(B, C, H, W, k, "smooth", seed=23)
-    ref_out, ref_gs, ref_gf, ref_gl = RC.local_attn_fwd_bwd(src, flow, logits, gout, k, chunk=1)
+    (src, flow, logits, gout), k = cfg2_case("fp32")
+    ref = _Ref(REF["fp32"])
     out = F_.local_attn_fwd(src, flow, logits, k)
     gs, gf, gl = F_.local_attn_bwd(src, flow, logits, gout, k)
-    assert (out - ref_out).abs().max().item() <= 1e-4
-    assert (gs - ref_gs).abs().max().item() <= 1e-4 * max(1.0, ref_gs.abs().max().item())
-    assert (gl - ref_gl).abs().max().item() <= 1e-4 * max(1.0, ref_gl.abs().max().item())
-    assert (gf - ref_gf).abs().max().item() <= 1e-4 * max(1.0, ref_gf.abs().max().item())
+    assert (_at(out) - ref["out"]).abs().max().item() <= 1e-4
+    assert (_at(gs) - ref["grad_source"]).abs().max().item() <= 1e-4 * max(1.0, ref.absmax("grad_source"))
+    assert (_at(gl) - ref["grad_logits"]).abs().max().item() <= 1e-4 * max(1.0, ref.absmax("grad_logits"))
+    assert (_at(gf) - ref["grad_flow"]).abs().max().item() <= 1e-4 * max(1.0, ref.absmax("grad_flow"))
 
 
-def test_cfg2_one_fullsize_sample_vs_host_reference(ref_lib, F_):
-    """...and one full-size sample against the HOST build of the reference bodies (all cores), forward + backward,
-    tile path: closes the chain without going through any GPU-side checker"""
-    import os
-    from oracle.ref_pipeline import local_attn_fwd_bwd
-    ref_lib.set_threads(max(1, (os.cpu_count() or 2) // 2))
-    B, C, H, W, k = 1, 256, 256, 256, 5
-    src, flow, logits, gout = _inputs(B, C, H, W, k, "smooth", seed=24)
+def test_cfg2_one_fullsize_sample_vs_host_reference(REF, F_):
+    """...and one more full-size sample, forward + backward, tile path"""
+    (src, flow, logits, gout), k = cfg2_case("host")
+    ref = _Ref(REF["host"])
     sb, lb, gb = src.bfloat16(), logits.bfloat16(), gout.bfloat16()
-    r_out, _, r_gs, r_gf, r_gl = local_attn_fwd_bwd(ref_lib, sb.float().cpu().numpy(), flow.cpu().numpy(), lb.float().cpu().numpy(),
-                                                    gb.float().cpu().numpy(), k)
-    ref_lib.set_threads(1)
     s_cl, g_cl = sb.contiguous(memory_format=CL), gb.contiguous(memory_format=CL)
     out = F_.local_attn_fwd(s_cl, flow, lb, k, algo="tile")
     gs, gf, gl = F_.local_attn_bwd(s_cl, flow, lb, g_cl, k, algo="tile")
-    t = lambda a: torch.from_numpy(a).to(DEV)
-    assert (out.float() - t(r_out)).abs().max().item() <= 1e-2
-    assert (gs.float() - t(r_gs)).abs().max().item() <= 1e-2
-    assert (gl.float() - t(r_gl)).abs().max().item() <= 1e-2
-    assert (gf - t(r_gf)).abs().max().item() <= 1e-2 * max(1.0, float(np.abs(r_gf).max()))
+    assert (_at(out) - ref["out"]).abs().max().item() <= 1e-2
+    assert (_at(gs) - ref["grad_source"]).abs().max().item() <= 1e-2
+    assert (_at(gl) - ref["grad_logits"]).abs().max().item() <= 1e-2
+    assert (_at(gf) - ref["grad_flow"]).abs().max().item() <= 1e-2 * max(1.0, ref.absmax("grad_flow"))
 
 
 # ----------------------------------------------------------------------------- unfused ops at (chunks of) their BASELINE sizes
-def test_block_extractor_cfg2_chunk_vs_reference_cuda(RC, F_):
-    B, C, H, W, k = 1, 256, 256, 256, 5
-    src, flow, _, _ = _inputs(B, C, H, W, k, "smooth", seed=25)
+def test_block_extractor_cfg2_chunk_vs_reference_cuda(REF, F_):
+    (src, flow, go), k = block_extractor_case()
+    ref = _Ref(REF["block_extractor"])
     ours = F_.block_extract_fwd(src, flow, k)
-    ref = RC.block_extract_fwd(src, flow, k)
-    assert (ours - ref).abs().max().item() <= 1e-5      # nvcc contracts the reference's mul+add chains, ours does not
-    del ours, ref
-    go = torch.randn(B, C, k * H, k * W, device=DEV)
+    assert (_at(ours) - ref["out"]).abs().max().item() <= 1e-5
+    del ours
     gs, gf = F_.block_extract_bwd(src, flow, go, k)
-    rgs, rgf = RC.block_extract_bwd(src, flow, go, k)
-    assert (gs - rgs).abs().max().item() <= 1e-4 * max(1.0, rgs.abs().max().item())
-    assert (gf - rgf).abs().max().item() <= 1e-4 * max(1.0, rgf.abs().max().item())
+    assert (_at(gs) - ref["grad_source"]).abs().max().item() <= 1e-4 * max(1.0, ref.absmax("grad_source"))
+    assert (_at(gf) - ref["grad_flow"]).abs().max().item() <= 1e-4 * max(1.0, ref.absmax("grad_flow"))
 
 
 @pytest.mark.parametrize("ks,sigma", [(2, 5.0), (4, 2.0)])
-def test_resample2d_cfg3_chunk_vs_reference_cuda(RC, F_, ks, sigma):
+def test_resample2d_cfg3_chunk_vs_reference_cuda(REF, F_, ks, sigma):
     """cfg3 shape (C=128, 512x512 fp32), two samples: forward and both gradients vs the reference's kernels"""
-    B, C, H, W = 2, 128, 512, 512
-    g = torch.Generator(device="cpu").manual_seed(31)
-    x = torch.randn(B, C, H, W, generator=g).to(DEV)
-    go = torch.randn(B, C, H, W, generator=g).to(DEV)
-    in2 = torch.cat([_smooth_flow(B, H, W, seed=3), torch.full((B, 1, H, W), sigma, device=DEV)], 1).contiguous()
+    (x, in2, go), ks = resample2d_case(ks, sigma)
+    ref = _Ref(REF[f"resample2d_ks{ks}"])
     out = F_.resample2d_fwd(x, in2, ks, 1)
-    ref = RC.resample2d_fwd(x, in2, ks, 1)
-    assert (out - ref).abs().max().item() <= 1e-4
+    assert (_at(out) - ref["out"]).abs().max().item() <= 1e-4
     g1, g2 = F_.resample2d_bwd(x, in2, go, ks, 1)
-    r1, r2 = RC.resample2d_bwd(x, in2, go, ks, 1)
-    assert (g1 - r1).abs().max().item() <= 1e-4 * max(1.0, r1.abs().max().item())
-    assert (g2 - r2).abs().max().item() <= 1e-4 * max(1.0, r2.abs().max().item())
+    assert (_at(g1) - ref["grad_in1"]).abs().max().item() <= 1e-4 * max(1.0, ref.absmax("grad_in1"))
+    assert (_at(g2) - ref["grad_in2"]).abs().max().item() <= 1e-4 * max(1.0, ref.absmax("grad_in2"))

@@ -4,11 +4,10 @@
 Oracles:
   * the CPU oracle's resample2d (forward and backward) composed with the cosine in numpy (float64 chain rule written out below);
   * the UNFUSED composition on the GPU: ``F.cosine_similarity(gfla_b200.Resample2d(...)(x, flow), target)`` with torch autograd;
-  * the reference's own ``PerceptualCorrectness`` class (byte-identical snapshot in baseline/_ref) on a shared random VGG19.
+  * the loss and flow gradients the reference's own ``PerceptualCorrectness`` class computed with the same feature extractor
+    (tests/golden/reference_perceptual.npz).
 Tolerances: fp32 1e-5 relative to the largest magnitude of the compared tensor, fp64 1e-11.
 """
-import sys
-import types
 
 import numpy as np
 import pytest
@@ -121,45 +120,29 @@ def test_resample2d_cosine_backward_skips_unrequested_gradients():
     assert flow.grad is not None and torch.isfinite(flow.grad).all()
 
 
-def test_perceptual_correctness_equals_reference_class(monkeypatch):
-    """the reference's PerceptualCorrectness (external_function.py:222-284, unmodified file from the snapshot) running on this
-    library's Resample2d, against gfla_b200.PerceptualCorrectness on the fused op: same VGG19 (random weights), same loss,
-    same flow gradients, with and without a mask"""
-    import bench_models
+def test_perceptual_correctness_equals_reference_class():
+    """the reference's PerceptualCorrectness (external_function.py:222-284) with its Resample2d(4, 1, sigma=2) against
+    gfla_b200.PerceptualCorrectness on the fused op: same feature extractor, same loss, same flow gradients, with and without
+    a mask.  The reference class's values (its resample op on the reference's kernel bodies) are stored in
+    tests/golden/reference_perceptual.npz by tests/golden/make_golden.py."""
     import gfla_b200
-    import torchvision
-    if bench_models.reference_root() is None:
-        pytest.skip("baseline/_ref snapshot of the reference not present")
-    bench_models.load_generators("literal")                       # compat.install(): reference modules on this library's ops
-    util = types.ModuleType("util")
-    util.util = types.ModuleType("util.util")                    # external_function.py:8 imports it for visualisation helpers only
-    sys.modules.setdefault("util", util)
-    sys.modules.setdefault("util.util", util.util)
-    orig = torchvision.models.vgg19
-    monkeypatch.setattr(torchvision.models, "vgg19", lambda pretrained=False, **kw: orig(weights=None))   # no network: random VGG
-    import importlib
-    ef = importlib.import_module("model.networks.external_function")
-    torch.manual_seed(0)
-    ref = ef.PerceptualCorrectness().to(DEV).eval()
-    ours = gfla_b200.PerceptualCorrectness(vgg=ref.vgg).to(DEV).eval()
-    B = 2
-    target = torch.rand(B, 3, 64, 64, device=DEV)
-    source = torch.rand(B, 3, 64, 64, device=DEV)
-    mask = (torch.rand(B, 1, 64, 64, device=DEV) > 0.4).float()
-    flows = [(torch.randn(B, 2, 8, 8, device=DEV) * 1.5), (torch.randn(B, 2, 16, 16, device=DEV) * 2.5)]
+    from conftest import FixedFeatures, load_golden, perceptual_inputs
+    ref = load_golden("reference_perceptual")
+    ours = gfla_b200.PerceptualCorrectness(vgg=FixedFeatures()).to(DEV).eval()
+    target, source, mask, flows = perceptual_inputs(DEV)
     old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
     torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False
     try:
-        for m in (None, mask):
-            fa = [f.clone().requires_grad_() for f in flows]
+        for name, m in (("nomask", None), ("mask", mask)):
+            want = ref[f"resample_{name}"]
             fb = [f.clone().requires_grad_() for f in flows]
-            la = ref(target, source, fa, [2, 3], m)
             lb = ours(target, source, fb, [2, 3], m)
-            assert abs(float(la) - float(lb)) <= 1e-5 * max(1.0, abs(float(la)))
-            la.backward()
+            la = float(want["loss"])
+            assert abs(la - float(lb)) <= 1e-5 * max(1.0, abs(la))
             lb.backward()
-            for a, b in zip(fa, fb):
-                assert a.grad.abs().max().item() > 0
-                assert (a.grad - b.grad).abs().max().item() <= 1e-4 * max(1e-6, a.grad.abs().max().item())
+            for i, b in enumerate(fb):
+                a = torch.from_numpy(want[f"grad{i}"]).to(DEV)
+                assert a.abs().max().item() > 0
+                assert (a - b.grad).abs().max().item() <= 1e-4 * max(1e-6, a.abs().max().item())
     finally:
         torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old

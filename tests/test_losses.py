@@ -67,41 +67,23 @@ def test_affine_regularization_gradient_and_multi_level():
     assert abs(float(multi([f3, f2])) - float(want)) < 1e-12
 
 
-def test_perceptual_correctness_bilinear_branch_equals_reference_class(monkeypatch):
-    """gfla_b200.PerceptualCorrectness vs the reference's class (external_function.py:222-320, unmodified snapshot file) on CPU
-    through the ``use_bilinear_sampling`` branch, which needs no custom op: everything around the fused resample -> cosine op
+def test_perceptual_correctness_bilinear_branch_equals_reference_class():
+    """gfla_b200.PerceptualCorrectness vs the reference's class (external_function.py:222-320) on CPU through the
+    ``use_bilinear_sampling`` branch, which needs no custom op: everything around the fused resample -> cosine op
     (correlation, max, loss map, mask handling, layer bookkeeping) is pinned here; the fused branch is pinned on the GPU
-    (tests/test_gpu_resample_cosine.py)."""
-    import importlib
-    import sys
-    import types
-    import torchvision
-    import bench_models
-    import gfla_b200
-    if bench_models.reference_root() is None:
-        pytest.skip("baseline/_ref snapshot of the reference not present")
-    bench_models.load_generators("literal")
-    util = types.ModuleType("util")
-    util.util = types.ModuleType("util.util")
-    sys.modules.setdefault("util", util)
-    sys.modules.setdefault("util.util", util.util)
-    orig = torchvision.models.vgg19
-    monkeypatch.setattr(torchvision.models, "vgg19", lambda pretrained=False, **kw: orig(weights=None))
-    ef = importlib.import_module("model.networks.external_function")
-    torch.manual_seed(0)
-    ref = ef.PerceptualCorrectness().eval()
-    ours = gfla_b200.PerceptualCorrectness(vgg=ref.vgg).eval()
-    B = 2
-    target, source = torch.rand(B, 3, 64, 64), torch.rand(B, 3, 64, 64)
-    mask = (torch.rand(B, 1, 64, 64) > 0.4).float()
-    flows = [torch.randn(B, 2, 8, 8) * 1.5, torch.randn(B, 2, 16, 16) * 2.5]
-    for m in (None, mask):
-        fa = [f.clone().requires_grad_() for f in flows]
+    (tests/test_gpu_resample_cosine.py).  The reference class's loss and flow gradients on these inputs, with the same
+    feature extractor, are stored in tests/golden/reference_perceptual.npz by tests/golden/make_golden.py."""
+    from conftest import FixedFeatures, load_golden, perceptual_inputs
+    ref = load_golden("reference_perceptual")
+    ours = gfla_b200.PerceptualCorrectness(vgg=FixedFeatures()).eval()
+    target, source, mask, flows = perceptual_inputs()
+    for name, m in (("nomask", None), ("mask", mask)):
+        want = ref[f"bilinear_{name}"]
         fb = [f.clone().requires_grad_() for f in flows]
-        la, lb = ref(target, source, fa, [2, 3], m, True), ours(target, source, fb, [2, 3], m, True)
-        assert abs(la.item() - lb.item()) <= 1e-6
-        la.backward()
+        lb = ours(target, source, fb, [2, 3], m, True)
+        assert abs(float(want["loss"]) - lb.item()) <= 1e-6
         lb.backward()
-        for a, b in zip(fa, fb):
-            assert a.grad.abs().max().item() > 1e-5
-            assert (a.grad - b.grad).abs().max().item() <= 1e-6 * max(1.0, a.grad.abs().max().item())
+        for i, b in enumerate(fb):
+            a = torch.from_numpy(want[f"grad{i}"])
+            assert a.abs().max().item() > 1e-5
+            assert (a - b.grad).abs().max().item() <= 1e-6 * max(1.0, a.abs().max().item())

@@ -7,7 +7,7 @@ vectorised softmax / avg_pool2d."""
 import numpy as np
 import pytest
 
-from conftest import load_golden
+from conftest import load_golden, sha256
 
 
 @pytest.mark.parametrize("case", sorted(load_golden("block_extractor")))
@@ -15,7 +15,7 @@ def test_block_extractor(oracle_lib, case):
     g = load_golden("block_extractor")[case]
     k = int(g["k"])
     out = oracle_lib.block_extract_fwd(g["source"], g["flow"], k)
-    assert np.array_equal(out, g["out"])
+    assert sha256(out) == str(g["out_sha256"])
     gs, gf = oracle_lib.block_extract_bwd(g["source"], g["flow"], g["grad_out"], k)
     assert np.array_equal(gs, g["grad_source"])
     assert np.array_equal(gf, g["grad_flow"])
