@@ -35,6 +35,10 @@ SIGNATURES = {
     "gfla_resample2d_bwd": [_vp] * 5 + [_i] * 10 + [_vp],
     "gfla_resample2d_cosine_fwd": [_vp] * 5 + [_i] * 8 + [ctypes.c_double, _i, _vp],
     "gfla_resample2d_cosine_bwd": [_vp] * 9 + [_i] * 8 + [ctypes.c_double, _i, _i, _vp],
+    "gfla_resample2d_fwd_nhwc": [_vp] * 3 + [_i] * 9 + [_vp],
+    "gfla_resample2d_bwd_nhwc": [_vp] * 5 + [_i] * 11 + [_vp],
+    "gfla_resample2d_cosine_fwd_nhwc": [_vp] * 5 + [_i] * 8 + [ctypes.c_double, _i, _vp],
+    "gfla_resample2d_cosine_bwd_nhwc": [_vp] * 9 + [_i] * 8 + [ctypes.c_double, _i, _i, _i, _vp],
     "gfla_local_attn_fwd": [_vp] * 5 + [_i] * 11 + [_vp],
     "gfla_local_attn_blend_fwd": [_vp] * 6 + [_i] * 11 + [_vp],
     "gfla_local_attn_bwd": [_vp] * 7 + [_i] * 12 + [_vp],

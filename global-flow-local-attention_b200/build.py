@@ -27,7 +27,7 @@ ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-I", INCLUDE]
 # per-file extras: the unfused ops keep IEEE mul/add separate so that their fp32 /
 # fp64 forward is bit-identical to the (uncontracted) CPU oracle.
-EXTRA = {"block_extract.cu": ["-fmad=false"], "resample2d.cu": ["-fmad=false"]}
+EXTRA = {"block_extract.cu": ["-fmad=false"], "resample2d.cu": ["-fmad=false"], "resample2d_nhwc.cu": ["-fmad=false"]}
 
 
 def _nvcc() -> str:

@@ -13,6 +13,11 @@ int resample2d_bwd(const void*, const void*, const void*, void*, void*, int, int
 int resample2d_cos_fwd(const void*, const void*, const void*, void*, void*, int, int, int, int, int, int, int, int, double, int, cudaStream_t);
 int resample2d_cos_bwd(const void*, const void*, const void*, const void*, const void*, void*, void*, void*, void*, int, int, int, int, int,
                        int, int, int, double, int, int, cudaStream_t);
+int resample2d_nhwc_fwd(const void*, const void*, void*, int, int, int, int, int, int, int, int, int, cudaStream_t);
+int resample2d_nhwc_bwd(const void*, const void*, const void*, void*, void*, int, int, int, int, int, int, int, int, int, int, int, cudaStream_t);
+int resample2d_nhwc_cos_fwd(const void*, const void*, const void*, void*, void*, int, int, int, int, int, int, int, int, double, int, cudaStream_t);
+int resample2d_nhwc_cos_bwd(const void*, const void*, const void*, const void*, const void*, void*, void*, void*, void*, int, int, int, int,
+                            int, int, int, int, double, int, int, int, cudaStream_t);
 int local_attn_fwd_gather(const void*, const void*, const void*, void*, void*, const void*, const void*, int, int, int, int, int, int, int, int, int, int, cudaStream_t);
 int local_attn_bwd_gather(const void*, const void*, const void*, const void*, void*, void*, void*, int, int, int, int, int, int, int, int, int, int, int, int, cudaStream_t);
 bool local_attn_bwd_tc_supported(int C, int k, int dtype, int flow_dtype, int layout, const void* gout, const void* gsrc);
@@ -49,6 +54,9 @@ constexpr bool kBwdFusedDefault = true;
 
 static inline bool pos(int a) { return a > 0; }
 static inline bool dtype_known(int d) { return elem_size(d) != 0; }
+static inline bool dtype_16bit(int d) { return d == GFLA_BF16 || d == GFLA_F16; }
+// grad_in1 of the channels-last 16-bit resample2d entries: the feature dtype, or fp32 (narrowed by the caller)
+static inline bool grad_in1_dtype_ok(int dtype, int gdtype) { return gdtype == dtype || gdtype == GFLA_F32; }
 
 extern "C" {
 
@@ -190,6 +198,53 @@ int gfla_resample2d_cosine_bwd(const void* in1, const void* in2, const void* tar
     if (grad_target != nullptr) { REQ_ALIGN(grad_target, dtype); }
     return resample2d_cos_bwd(in1, in2, target, stats, grad_cos, grad_in1, grad_in2, grad_val, grad_target, B, C, Hi, Wi, H, W, ks, dilation,
                               eps, dtype, accumulate, (cudaStream_t)stream);
+}
+
+int gfla_resample2d_fwd_nhwc(const void* in1, const void* in2, void* out, int B, int C, int Hi, int Wi, int H, int W, int ks,
+                             int dilation, int dtype, gfla_stream_t stream) {
+    REQ_PTR(in1); REQ_PTR(in2); REQ_PTR(out);
+    if (!pos(B) || !pos(C) || !pos(Hi) || !pos(Wi) || !pos(H) || !pos(W) || ks < 2 || ks > 9 || dilation < 1) return GFLA_E_SHAPE;
+    if (!dtype_16bit(dtype)) return GFLA_E_DTYPE;
+    REQ_ALIGN(in1, dtype); REQ_ALIGN(in2, GFLA_F32); REQ_ALIGN(out, dtype);
+    return resample2d_nhwc_fwd(in1, in2, out, B, C, Hi, Wi, H, W, ks, dilation, dtype, (cudaStream_t)stream);
+}
+
+int gfla_resample2d_bwd_nhwc(const void* in1, const void* in2, const void* grad_out, void* grad_in1, void* grad_in2, int B, int C,
+                             int Hi, int Wi, int H, int W, int ks, int dilation, int dtype, int grad_in1_dtype, int accumulate,
+                             gfla_stream_t stream) {
+    REQ_PTR(in1); REQ_PTR(in2); REQ_PTR(grad_out); REQ_PTR(grad_in1); REQ_PTR(grad_in2);
+    if (!pos(B) || !pos(C) || !pos(Hi) || !pos(Wi) || !pos(H) || !pos(W) || ks < 2 || ks > 9 || dilation < 1) return GFLA_E_SHAPE;
+    if (!dtype_16bit(dtype) || !grad_in1_dtype_ok(dtype, grad_in1_dtype)) return GFLA_E_DTYPE;
+    REQ_ALIGN(in1, dtype); REQ_ALIGN(in2, GFLA_F32); REQ_ALIGN(grad_out, dtype); REQ_ALIGN(grad_in1, grad_in1_dtype);
+    REQ_ALIGN(grad_in2, GFLA_F32);
+    return resample2d_nhwc_bwd(in1, in2, grad_out, grad_in1, grad_in2, B, C, Hi, Wi, H, W, ks, dilation, dtype, grad_in1_dtype,
+                               accumulate, (cudaStream_t)stream);
+}
+
+int gfla_resample2d_cosine_fwd_nhwc(const void* in1, const void* in2, const void* target, void* cos_out, void* stats, int B, int C,
+                                    int Hi, int Wi, int H, int W, int ks, int dilation, double eps, int dtype, gfla_stream_t stream) {
+    REQ_PTR(in1); REQ_PTR(in2); REQ_PTR(target); REQ_PTR(cos_out); REQ_PTR(stats);
+    if (!pos(B) || !pos(C) || !pos(Hi) || !pos(Wi) || !pos(H) || !pos(W) || ks < 2 || ks > 9 || dilation < 1 || !(eps >= 0)) return GFLA_E_SHAPE;
+    if (!dtype_16bit(dtype)) return GFLA_E_DTYPE;
+    REQ_ALIGN(in1, dtype); REQ_ALIGN(target, dtype); REQ_ALIGN(in2, GFLA_F32); REQ_ALIGN(cos_out, GFLA_F32); REQ_ALIGN(stats, GFLA_F32);
+    return resample2d_nhwc_cos_fwd(in1, in2, target, cos_out, stats, B, C, Hi, Wi, H, W, ks, dilation, eps, dtype, (cudaStream_t)stream);
+}
+
+int gfla_resample2d_cosine_bwd_nhwc(const void* in1, const void* in2, const void* target, const void* stats, const void* grad_cos,
+                                    void* grad_in1, void* grad_in2, void* grad_val, void* grad_target, int B, int C, int Hi, int Wi,
+                                    int H, int W, int ks, int dilation, double eps, int dtype, int grad_in1_dtype, int accumulate,
+                                    gfla_stream_t stream) {
+    REQ_PTR(in1); REQ_PTR(in2); REQ_PTR(target); REQ_PTR(stats); REQ_PTR(grad_cos); REQ_PTR(grad_in2);
+    if (grad_in1 != nullptr && grad_val == nullptr) return GFLA_E_NULL;      // the scatter runs on the materialised d/d(warped)
+    if (!pos(B) || !pos(C) || !pos(Hi) || !pos(Wi) || !pos(H) || !pos(W) || ks < 2 || ks > 9 || dilation < 1 || !(eps >= 0)) return GFLA_E_SHAPE;
+    if (!dtype_16bit(dtype) || !grad_in1_dtype_ok(dtype, grad_in1_dtype)) return GFLA_E_DTYPE;
+    REQ_ALIGN(in1, dtype); REQ_ALIGN(target, dtype); REQ_ALIGN(in2, GFLA_F32); REQ_ALIGN(stats, GFLA_F32); REQ_ALIGN(grad_cos, GFLA_F32);
+    REQ_ALIGN(grad_in2, GFLA_F32);
+    if (grad_in1 != nullptr) { REQ_ALIGN(grad_in1, grad_in1_dtype); }
+    if (grad_val != nullptr) { REQ_ALIGN(grad_val, dtype); }
+    if (grad_target != nullptr) { REQ_ALIGN(grad_target, dtype); }
+    return resample2d_nhwc_cos_bwd(in1, in2, target, stats, grad_cos, grad_in1, grad_in2, grad_val, grad_target, B, C, Hi, Wi, H, W, ks,
+                                   dilation, eps, dtype, grad_in1_dtype, accumulate, (cudaStream_t)stream);
 }
 
 static int local_attn_fwd_any(const void* source, const void* flow, const void* logits, void* out, void* probs,

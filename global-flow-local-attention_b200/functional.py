@@ -120,6 +120,10 @@ def attn_reshape_bwd(grad_out: torch.Tensor, k: int, grad_in=None) -> torch.Tens
 
 # --------------------------------------------------------------------------- resample2d
 def resample2d_fwd(input1: torch.Tensor, input2: torch.Tensor, kernel_size: int, dilation: int) -> torch.Tensor:
+    """fp32 / fp64: planar kernels, input2 in input1's dtype.  bf16 / fp16: channels-last kernels, input2 fp32; input1 may be
+    channels_last (used as it is) or contiguous NCHW (re-laid), and the output comes back in input1's memory format."""
+    if input1.dtype in _HALF:
+        return _resample2d_fwd_16(input1, input2, kernel_size, dilation)
     assert input1.is_contiguous() and input2.is_contiguous()
     _need_cuda(input1, input2)
     _, d, hi, wi = input1.size()
@@ -135,6 +139,8 @@ def resample2d_fwd(input1: torch.Tensor, input2: torch.Tensor, kernel_size: int,
 
 
 def resample2d_bwd(input1, input2, grad_out, kernel_size, dilation, grad_input1=None, grad_input2=None):
+    if input1.dtype in _HALF:
+        return _resample2d_bwd_16(input1, input2, grad_out, kernel_size, dilation, grad_input1, grad_input2)
     assert input1.is_contiguous() and input2.is_contiguous()
     grad_out = grad_out.contiguous()
     _need_cuda(input1, input2, grad_out)
@@ -152,7 +158,11 @@ def resample2d_bwd(input1, input2, grad_out, kernel_size, dilation, grad_input1=
 
 def resample2d_cosine_fwd(input1, input2, target, kernel_size: int, dilation: int, eps: float = 1e-8):
     """cos[b,y,x] = cosine_similarity(resample2d(input1, input2)[b,:,y,x], target[b,:,y,x]) without the warped tensor
-    (external_function.py:275-279).  -> (cos [B,H,W], stats [B,3,H,W] for the backward)"""
+    (external_function.py:275-279).  -> (cos [B,H,W], stats [B,3,H,W] for the backward)
+    bf16 / fp16 features (input1, target; channels_last or NCHW) take the channels-last kernels with an fp32 input2, and
+    cos / stats are fp32."""
+    if input1.dtype in _HALF:
+        return _resample2d_cosine_fwd_16(input1, input2, target, kernel_size, dilation, eps)
     assert input1.is_contiguous() and input2.is_contiguous() and target.is_contiguous()
     _need_cuda(input1, input2, target)
     _, d, hi, wi = input1.size()
@@ -173,6 +183,9 @@ def resample2d_cosine_fwd(input1, input2, target, kernel_size: int, dilation: in
 def resample2d_cosine_bwd(input1, input2, target, stats, grad_cos, kernel_size, dilation, eps=1e-8, need_input1=False,
                           need_target=False):
     """-> (grad_input1 | None, grad_input2, grad_target | None)"""
+    if input1.dtype in _HALF:
+        return _resample2d_cosine_bwd_16(input1, input2, target, stats, grad_cos, kernel_size, dilation, eps, need_input1,
+                                         need_target)
     grad_cos = grad_cos.contiguous()
     _need_cuda(input1, input2, target, stats, grad_cos)
     _, d, hi, wi = input1.size()
@@ -186,6 +199,129 @@ def resample2d_cosine_bwd(input1, input2, target, stats, grad_cos, kernel_size, 
             _p(input1), _p(input2), _p(target), _p(stats), _p(grad_cos), _p(grad_in1) if need_input1 else None, _p(grad_in2),
             _p(grad_val) if need_input1 else None, _p(grad_target) if need_target else None, b, d, hi, wi, h, w, kernel_size, dilation,
             float(eps), _dt(input1), 0, _stream(input1)), "resample2d_cosine_bwd")
+    return grad_in1, grad_in2, grad_target
+
+
+# --------------------------------------------------------------------------- resample2d, 16-bit channels-last
+_HALF = (torch.bfloat16, torch.float16)
+
+
+def flow_f32(features: torch.Tensor, flow: torch.Tensor) -> torch.Tensor:
+    """16-bit feature tensors pair with an fp32 flow: the tap indices and weights are then bit-identical to the fp32
+    path (block_extractor_kernel.cu:62-76, resample2d_kernel.cu:43-60), and the tcgen05 tile kernels -- which take fp32
+    flow only -- serve the call.  A bf16/f16 flow (e.g. from a network cast wholesale with .bfloat16()) is widened here;
+    autograd casts its gradient back to the flow's dtype."""
+    if features.dtype in _HALF and flow.dtype != torch.float32:
+        return flow.float()
+    return flow
+
+
+def _to_nhwc(t: torch.Tensor) -> torch.Tensor:
+    """a [B,C,H,W] tensor in channels-last storage: as it is when it already is, re-laid by the library when it is NCHW"""
+    if t.is_contiguous(memory_format=torch.channels_last):
+        return t
+    return relayout(t.contiguous(), True)
+
+
+def _like_caller(t: torch.Tensor, planar: bool) -> torch.Tensor:
+    """a channels-last result back in the caller's memory format (planar = the caller's tensor was contiguous NCHW)"""
+    return relayout(t, False) if planar and not t.is_contiguous() else t
+
+
+def _narrow(t: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
+    """fp32 -> 16-bit copy of a dense (NCHW or channels-last) tensor with the library's kernel, keeping its strides"""
+    out = torch.empty_like(t, dtype=dtype)
+    with torch.cuda.device_of(t):
+        _lib.check(_lib.lib().gfla_convert(_p(t), _dt(t), _p(out), _DT[dtype], t.numel(), _stream(t)), "convert")
+    return out
+
+
+def _in2_f32(input2: torch.Tensor) -> None:
+    assert input2.is_contiguous()
+    b, three, h, w = input2.size()
+    assert three == 3, "input2 must be [B,3,H,W] = (dx, dy, sigma) (resample2d.py:51-52)"
+    if input2.dtype != torch.float32:
+        raise TypeError("resample2d: bfloat16/float16 input1 takes a float32 input2 (dx, dy, sigma)")
+
+
+def _resample2d_fwd_16(input1, input2, kernel_size, dilation):
+    _in2_f32(input2)
+    _need_cuda(input1, input2)
+    planar = input1.is_contiguous()
+    x = _to_nhwc(input1)
+    _, d, hi, wi = x.size()
+    b, _, h, w = input2.size()
+    out = torch.empty((b, d, h, w), dtype=x.dtype, device=x.device, memory_format=torch.channels_last)
+    with torch.cuda.device_of(x):
+        _lib.check(_lib.lib().gfla_resample2d_fwd_nhwc(_p(x), _p(input2), _p(out), b, d, hi, wi, h, w, kernel_size, dilation, _dt(x),
+                                                       _stream(x)), "resample2d_fwd_nhwc")
+    return _like_caller(out, planar)
+
+
+def _resample2d_bwd_16(input1, input2, grad_out, kernel_size, dilation, grad_input1=None, grad_input2=None):
+    """grad_input1 comes back in input1's dtype and memory format, grad_input2 in fp32.  Buffers passed in (reference
+    contract: gradients are ADDED) must be channels_last for grad_input1 (its dtype or fp32) and fp32 for grad_input2."""
+    _in2_f32(input2)
+    _need_cuda(input1, input2, grad_out)
+    planar = input1.is_contiguous()
+    x, go = _to_nhwc(input1), _to_nhwc(grad_out)
+    _, d, hi, wi = x.size()
+    b, _, h, w = input2.size()
+    accumulate, narrow = 1, False
+    if grad_input1 is None:
+        # scatter into an fp32 buffer (fp32 reductions in L2) and narrow afterwards, as block_extract_bwd does
+        accumulate, narrow = 0, True
+        grad_input1 = torch.empty(x.shape, dtype=torch.float32, device=x.device, memory_format=torch.channels_last)
+        grad_input2 = torch.empty_like(input2)
+    assert grad_input1.is_contiguous(memory_format=torch.channels_last), "grad_input1 buffer must be channels_last"
+    assert grad_input2.is_contiguous() and grad_input2.dtype == torch.float32
+    with torch.cuda.device_of(x):
+        _lib.check(_lib.lib().gfla_resample2d_bwd_nhwc(_p(x), _p(input2), _p(go), _p(grad_input1), _p(grad_input2), b, d, hi, wi, h, w,
+                                                       kernel_size, dilation, _dt(x), _dt(grad_input1), accumulate, _stream(x)),
+                   "resample2d_bwd_nhwc")
+    if narrow:
+        grad_input1 = _like_caller(_narrow(grad_input1, x.dtype), planar)
+    return grad_input1, grad_input2
+
+
+def _resample2d_cosine_fwd_16(input1, input2, target, kernel_size, dilation, eps):
+    _in2_f32(input2)
+    _need_cuda(input1, input2, target)
+    if target.dtype != input1.dtype:
+        raise TypeError("resample2d_cosine: input1 and target must share a dtype")
+    x, tg = _to_nhwc(input1), _to_nhwc(target)
+    _, d, hi, wi = x.size()
+    b, _, h, w = input2.size()
+    assert tuple(tg.shape) == (b, d, h, w), "target must be [B,C,H,W] on the flow's grid"
+    cos = torch.empty((b, h, w), dtype=torch.float32, device=x.device)
+    stats = torch.empty((b, 3, h, w), dtype=torch.float32, device=x.device)
+    with torch.cuda.device_of(x):
+        _lib.check(_lib.lib().gfla_resample2d_cosine_fwd_nhwc(_p(x), _p(input2), _p(tg), _p(cos), _p(stats), b, d, hi, wi, h, w,
+                                                              kernel_size, dilation, float(eps), _dt(x), _stream(x)),
+                   "resample2d_cosine_fwd_nhwc")
+    return cos, stats
+
+
+def _resample2d_cosine_bwd_16(input1, input2, target, stats, grad_cos, kernel_size, dilation, eps, need_input1, need_target):
+    _in2_f32(input2)
+    grad_cos = grad_cos.float().contiguous()
+    _need_cuda(input1, input2, target, stats, grad_cos)
+    x, tg = _to_nhwc(input1), _to_nhwc(target)
+    _, d, hi, wi = x.size()
+    b, _, h, w = input2.size()
+    cl = torch.channels_last
+    grad_in2 = torch.empty_like(input2)
+    grad_in1 = torch.empty(x.shape, dtype=torch.float32, device=x.device, memory_format=cl) if need_input1 else None
+    grad_val = torch.empty(tg.shape, dtype=x.dtype, device=x.device, memory_format=cl) if need_input1 else None
+    grad_target = torch.empty(tg.shape, dtype=x.dtype, device=x.device, memory_format=cl) if need_target else None
+    with torch.cuda.device_of(x):
+        _lib.check(_lib.lib().gfla_resample2d_cosine_bwd_nhwc(
+            _p(x), _p(input2), _p(tg), _p(stats), _p(grad_cos), _p(grad_in1), _p(grad_in2), _p(grad_val), _p(grad_target), b, d, hi,
+            wi, h, w, kernel_size, dilation, float(eps), _dt(x), _lib.GFLA_F32, 0, _stream(x)), "resample2d_cosine_bwd_nhwc")
+    if need_input1:
+        grad_in1 = _like_caller(_narrow(grad_in1, x.dtype), input1.is_contiguous())
+    if need_target:
+        grad_target = _like_caller(grad_target, target.is_contiguous())
     return grad_in1, grad_in2, grad_target
 
 

@@ -6,12 +6,35 @@ from torch.nn.modules.module import Module
 from . import functional as F_
 
 
+def _features(t):
+    """16-bit channels_last feature maps stay as they are (the channels-last kernels read them in place); anything else
+    is made contiguous, as the reference's module does"""
+    if t.dtype in F_._HALF and t.dim() == 4 and t.is_contiguous(memory_format=torch.channels_last):
+        return t
+    return t.contiguous()
+
+
+def _input2(input1, flow, sigma):
+    """input2 = cat(flow, sigma plane) (resample2d.py:51-52) in the dtype the kernels take it in: fp32 next to bf16 / fp16
+    features (F_.flow_f32), input1's own dtype next to fp32 / fp64 ones (a bf16 generator's flow into an fp32 VGG).
+    Autograd casts the flow gradient back to the flow's dtype."""
+    flow = F_.flow_f32(input1, flow)
+    if flow.dtype != input1.dtype and input1.dtype not in F_._HALF:
+        flow = flow.to(input1.dtype)
+    plane = torch.full((flow.size(0), 1, flow.size(2), flow.size(3)), sigma, dtype=flow.dtype, device=flow.device)
+    return torch.cat((flow, plane), 1)
+
+
+def _is_features(t):
+    return t.is_contiguous() or (t.dtype in F_._HALF and t.dim() == 4 and t.is_contiguous(memory_format=torch.channels_last))
+
+
 class Resample2dFunction(Function):
     """reference: resample2d.py:6-39.  input2 carries (dx, dy, sigma)."""
 
     @staticmethod
     def forward(ctx, input1, input2, kernel_size=2, dilation=1):
-        assert input1.is_contiguous()
+        assert _is_features(input1)          # contiguous; bf16 / fp16 may also be channels_last
         assert input2.is_contiguous()
         ctx.save_for_backward(input1, input2)
         ctx.kernel_size = kernel_size
@@ -40,11 +63,8 @@ class Resample2d(Module):
         self.sigma = float(sigma)
 
     def forward(self, input1, input2):
-        input1_c = input1.contiguous()
-        sigma = torch.full((input2.size(0), 1, input2.size(2), input2.size(3)), self.sigma,
-                           dtype=input2.dtype, device=input2.device)
-        input2 = torch.cat((input2, sigma), 1)
-        return Resample2dFunction.apply(input1_c, input2, self.kernel_size, self.dilation)
+        input1_c = _features(input1)
+        return Resample2dFunction.apply(input1_c, _input2(input1_c, input2, self.sigma), self.kernel_size, self.dilation)
 
 
 class Resample2dCosineFunction(Function):
@@ -54,9 +74,9 @@ class Resample2dCosineFunction(Function):
 
     @staticmethod
     def forward(ctx, input1, input2, target, kernel_size=2, dilation=1, eps=1e-8):
-        assert input1.is_contiguous()
+        assert _is_features(input1)
         assert input2.is_contiguous()
-        target = target.contiguous()
+        target = _features(target)
         cos, stats = F_.resample2d_cosine_fwd(input1, input2, target, kernel_size, dilation, eps)
         ctx.save_for_backward(input1, input2, target, stats)
         ctx.cfg = (kernel_size, dilation, eps)
@@ -83,6 +103,6 @@ class Resample2dCosine(Module):
         self.eps = float(eps)
 
     def forward(self, input1, input2, target):
-        sigma = torch.full((input2.size(0), 1, input2.size(2), input2.size(3)), self.sigma, dtype=input2.dtype, device=input2.device)
-        input2 = torch.cat((input2, sigma), 1)
-        return Resample2dCosineFunction.apply(input1.contiguous(), input2, target, self.kernel_size, self.dilation, self.eps)
+        input1_c = _features(input1)
+        return Resample2dCosineFunction.apply(input1_c, _input2(input1_c, input2, self.sigma), target, self.kernel_size, self.dilation,
+                                              self.eps)

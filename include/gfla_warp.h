@@ -142,7 +142,8 @@ int gfla_attn_reshape_bwd(const void* grad_out, void* grad_in, int B, int H, int
  *   in1 [B,C,Hi,Wi]; in2 [B,3,H,W] = (dx, dy, sigma) -- the sigma plane is
  *   appended by the Python module (resample2d.py:51-52); out [B,C,H,W];
  *   grad_in2 [B,3,H,W] (all three planes are written, like :328).
- *   in2 / grad_in2 have the same dtype as in1 (F32 or F64 only).
+ *   in2 / grad_in2 have the same dtype as in1 (F32 or F64 only here; BF16 / F16
+ *   feature maps take the *_nhwc entries below).
  * ------------------------------------------------------------------------ */
 int gfla_resample2d_fwd(const void* in1, const void* in2, void* out,
                         int B, int C, int Hi, int Wi, int H, int W, int ks, int dilation,
@@ -168,7 +169,8 @@ int gfla_resample2d_bwd(const void* in1, const void* in2, const void* grad_out,
  *   grad_target [B,C,H,W] optional (NULL = not wanted);
  *   grad_in1 [B,C,Hi,Wi] optional -- it needs grad_val, a caller-provided
  *   [B,C,H,W] scratch tensor that receives d/d(warped) before the scatter.
- *   accumulate applies to grad_in1 / grad_in2 / grad_target.  F32 or F64.
+ *   accumulate applies to grad_in1 / grad_in2 / grad_target.  F32 or F64 here;
+ *   BF16 / F16 feature maps take the *_nhwc entries below.
  * ------------------------------------------------------------------------ */
 int gfla_resample2d_cosine_fwd(const void* in1, const void* in2, const void* target,
                                void* cos_out, void* stats,
@@ -179,6 +181,37 @@ int gfla_resample2d_cosine_bwd(const void* in1, const void* in2, const void* tar
                                void* grad_in1, void* grad_in2, void* grad_val, void* grad_target,
                                int B, int C, int Hi, int Wi, int H, int W, int ks, int dilation,
                                double eps, int dtype, int accumulate, gfla_stream_t stream);
+
+/* ------------------------------------------------------------------------ *
+ * resample2d and resample2d -> cosine on channels-last 16-bit feature maps
+ *   the same four operations as gfla_resample2d_{fwd,bwd} (resample2d_cuda.cc:6-33,
+ *   resample2d_kernel.cu:20-95, :98-202, :204-330) and gfla_resample2d_cosine_{fwd,bwd}
+ *   (external_function.py:275-279), for BF16 / F16 feature storage (`dtype`) in
+ *   NHWC = torch.channels_last order: in1 [B,Hi,Wi,C]; out, grad_out, target,
+ *   grad_val, grad_target [B,H,W,C]; grad_in1 [B,Hi,Wi,C].
+ *   in2 / grad_in2 [B,3,H,W], cos_out / grad_cos [B,H,W] and stats [B,3,H,W] are
+ *   planar F32.  Arithmetic is fp32: a pixel's taps and weights are those of the
+ *   F32 entries; sums over channels are fp32 in another order.
+ *   grad_in1_dtype: == dtype (16-bit reductions, each add rounded), or GFLA_F32
+ *   (fp32 reductions; narrow with gfla_convert()).  grad_val has `dtype`.
+ * ------------------------------------------------------------------------ */
+int gfla_resample2d_fwd_nhwc(const void* in1, const void* in2, void* out,
+                             int B, int C, int Hi, int Wi, int H, int W, int ks, int dilation,
+                             int dtype, gfla_stream_t stream);
+int gfla_resample2d_bwd_nhwc(const void* in1, const void* in2, const void* grad_out,
+                             void* grad_in1, void* grad_in2,
+                             int B, int C, int Hi, int Wi, int H, int W, int ks, int dilation,
+                             int dtype, int grad_in1_dtype, int accumulate, gfla_stream_t stream);
+int gfla_resample2d_cosine_fwd_nhwc(const void* in1, const void* in2, const void* target,
+                                    void* cos_out, void* stats,
+                                    int B, int C, int Hi, int Wi, int H, int W, int ks, int dilation,
+                                    double eps, int dtype, gfla_stream_t stream);
+int gfla_resample2d_cosine_bwd_nhwc(const void* in1, const void* in2, const void* target,
+                                    const void* stats, const void* grad_cos,
+                                    void* grad_in1, void* grad_in2, void* grad_val, void* grad_target,
+                                    int B, int C, int Hi, int Wi, int H, int W, int ks, int dilation,
+                                    double eps, int dtype, int grad_in1_dtype, int accumulate,
+                                    gfla_stream_t stream);
 
 /* ------------------------------------------------------------------------ *
  * fused local attention = the tail of ExtractorAttn.forward
